@@ -8,16 +8,18 @@
   --config 3            configs[2]: 1241x376 stereo pairs (KITTI shape), 2000 kp: extract L + R, stereo::compute, pose_optimizer
   --config 5            configs[4]: 1920x1080 perspective, 2000 kp, the config-4 pipeline, one stream per GPU
 
-One "step" = `frames_per_step` frames through the hot path on each of the --streams independent camera streams of a GPU
-(every stream owns its handles, CUDA streams and host thread; frames_per_step is calibrated in the warm-up so that the
-timed region lasts >= ~2 s and is reported in `config`).  Two measurements per run, over the SAME calls:
+One "step" = --frames-per-step frames (default 8) through the hot path on each of the --streams independent camera streams
+of a GPU (every stream owns its handles, CUDA streams and host thread); --warmup W (at least 3) untimed steps precede the
+--steps K timed ones.  Two measurements per run, over the SAME calls:
   value  every input already resident in HBM when the timed region starts (frames, BA graph): ovs_extract_device,
          ovs_robust_brute_force_match_device, ovs_frame_index_create_device, ovs_local_ba_prepare_device / run / fetch_device.
          The whole path is inside the timed region -- graph preparation, greedy replays, Levenberg loop -- only the
          host<->device copies of the inputs / results are not.
   e2e    the host-buffer C-ABI entry points a reference caller would use, every host<->device copy inside the timed region.
 `--impl reference` times the CPU oracle (the restated reference; the real one cannot be built here, see DESIGN.md) on the
-same workload with all usable host cores, as independent streams.  Prints ONE JSON line on rank 0."""
+same workload with all usable host cores, as independent streams.  Prints ONE JSON line on rank 0.
+`--dump-outputs DIR` writes what the value leg returned for the last frame of each camera stream as DIR/stream<k>_<name>.npy
+(float32 / float64); the inputs depend only on the arguments, so two builds can be compared output for output."""
 import argparse
 import ctypes as C
 import json
@@ -235,6 +237,7 @@ class CameraStream:
             self.d_ba_out = (torch.zeros_like(self.d_ba["poses"]), torch.zeros_like(self.d_ba["points"]),
                              torch.zeros(len(ba["obs_kf"]), dtype=torch.uint8, device=dev))
         self.n_prev, self.prev_desc, self.prev_kps = 0, None, None
+        self.last = {}                                 # host-side results of the last step_device frame (outputs())
         self.stage_ms = {"device": np.zeros(len(STAGES)), "host": np.zeros(len(STAGES))}
         self.reset()
 
@@ -252,16 +255,16 @@ class CameraStream:
         return s, xy
 
     def _common_tail(self, leg, fidx, n, i, t):
-        """projection match (+ pose optimiser, local BA) of frame i on the frame index `fidx`; t = stage clock list."""
-        cfg, pose = self.cfg, self.wl["pose"]
+        """projection match of frame i on the frame index `fidx` -> the matched landmark of every keypoint (-1: none); t = stage clock list."""
+        cfg = self.cfg
         s, xy = self._landmarks(i)
         if cfg["ba"]:
-            self.pj.match_frame_and_landmarks(fidx, self.sf, xy, None, s["level"], s["desc"], None, None, 5.0)
+            _, matched = self.pj.match_frame_and_landmarks(fidx, self.sf, xy, None, s["level"], s["desc"], None, None, 5.0)
         else:
-            self.pj.match_current_and_last_frames(fidx, self.sf, 8, np.ones(len(xy), np.uint8), xy, None, s["level"], s["angle"], s["desc"], None, 20.0)
+            _, matched = self.pj.match_current_and_last_frames(fidx, self.sf, 8, np.ones(len(xy), np.uint8), xy, None, s["level"], s["angle"], s["desc"], None, 20.0)
         fidx.close()
         t.append(time.perf_counter())
-        return pose
+        return matched
 
     def step_device(self, i):
         i = (i + 11 * self.sid) % self.ring            # streams walk the shared frame ring at different offsets
@@ -275,27 +278,32 @@ class CameraStream:
             nr = self.ext_r.extract_device(self.d_frames_r[i].data_ptr(), W, H, W, self.d_kps_r.data_ptr(), self.d_desc_r.data_ptr(), self.cap)
         t.append(time.perf_counter())
         pose = self.wl["pose"]
+        last = {"frame": i, "num_keypoints": n}
         if cfg["stereo"]:
+            last["num_keypoints_right"] = nr
             # stereo::compute takes the keypoint / descriptor arrays of both images (the API of the reference): they come to the
             # host once, the pyramids stay on the device
             kl = self.d_kps[cur][:n].cpu().numpy().view(self._kp_dtype()).reshape(-1); dl = self.d_desc[cur][:n].cpu().numpy()
             kr = self.d_kps_r[:nr].cpu().numpy().view(self._kp_dtype()).reshape(-1); dr = self.d_desc_r[:nr].cpu().numpy()
-            self.st.compute(self.ext, self.ext_r, kl, dl, kr, dr, pose["cam"]["focal_x_baseline"], pose["cam"]["focal_x_baseline"] / pose["cam"]["fx"])
+            last["stereo_x_right"], last["stereo_depth"], _ = self.st.compute(self.ext, self.ext_r, kl, dl, kr, dr, pose["cam"]["focal_x_baseline"],
+                                                                              pose["cam"]["focal_x_baseline"] / pose["cam"]["fx"])
             t.append(time.perf_counter())
             stages = ["extract", "stereo_match"]
         else:
             stages = ["extract"]
             if cfg["ba"]:
                 if self.n_prev:
-                    self.mt.brute_force_match_device(self.d_desc[cur].data_ptr(), n, self.d_desc[cur ^ 1].data_ptr(), self.n_prev)
+                    last["brute_force_matches"] = self.mt.brute_force_match_device(self.d_desc[cur].data_ptr(), n, self.d_desc[cur ^ 1].data_ptr(), self.n_prev)
                     sd["match_us"] += self.mt.last_kernel_us(); sd["match_calls"] += 1
                 self.n_prev = n
                 t.append(time.perf_counter()); stages.append("brute_force_match")
             from openvslam_b200 import match
             fidx = match.frame_index.from_device(self.pj, n, self.d_kps[cur].data_ptr(), self.d_desc[cur].data_ptr(), self.grid)
-            self._common_tail("device", fidx, n, i, t); stages.append("projection_match")
+            last["projection_matches"] = self._common_tail("device", fidx, n, i, t); stages.append("projection_match")
         xr = pose["obs_xr"] if cfg["stereo"] else None
-        _, _, _, pst = self.po.optimize(self.pcam, not cfg["stereo"], pose["pts_w"], pose["obs_xy"], xr, pose["inv_sigma_sq"], pose["poses"][0])
+        _, last["pose"], last["pose_outliers"], pst = self.po.optimize(self.pcam, not cfg["stereo"], pose["pts_w"], pose["obs_xy"], xr, pose["inv_sigma_sq"],
+                                                                        pose["poses"][0])
+        self.last = last
         sd["pose_us"] += pst["device_us"]
         t.append(time.perf_counter()); stages.append("pose_optimizer")
         if cfg["ba"]:
@@ -358,6 +366,27 @@ class CameraStream:
         from openvslam_b200 import feature
         return feature.KEYPOINT_DTYPE
 
+    def outputs(self):
+        """What the last step_device frame handed its caller, as float32 / float64 host arrays by name: keypoints (x, y, size,
+        angle, response, octave per row), descriptors (one byte value per column), match results (-1: no match), the optimised
+        pose and its outlier flags, and the local BA's poses, points and outlier flags."""
+        last = dict(self.last)
+        cur = last.pop("frame") & 1
+
+        def keypoints(d_kps, d_desc, n):
+            k = d_kps[:n].cpu().numpy().view(self._kp_dtype()).reshape(-1)
+            return (np.stack([k[f].astype(np.float32) for f in ("x", "y", "size", "angle", "response", "octave")], 1),
+                    d_desc[:n].cpu().numpy().astype(np.float32))
+        out = dict(zip(("keypoints", "descriptors"), keypoints(self.d_kps[cur], self.d_desc[cur], last.pop("num_keypoints"))))
+        if "num_keypoints_right" in last:
+            out.update(zip(("keypoints_right", "descriptors_right"), keypoints(self.d_kps_r, self.d_desc_r, last.pop("num_keypoints_right"))))
+        if self.cfg["ba"]:
+            last.update(zip(("local_ba_poses", "local_ba_points", "local_ba_outliers"), (a.cpu().numpy() for a in self.d_ba_out)))
+        for name, a in last.items():
+            a = np.asarray(a)
+            out[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+        return out
+
     def bytes_per_frame(self):
         """host<->device bytes of one e2e frame, counted from the arrays the host entry points copy."""
         cfg, pose = self.cfg, self.wl["pose"]
@@ -386,6 +415,24 @@ class CameraStream:
         for h in (self.ext, self.ext_r, self.mt, self.pj, self.st, self.po, getattr(self, "lba", None), getattr(self, "pba", None)):
             if h is not None:
                 h.close()
+
+
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_outputs(cams, path):
+    """Writes CameraStream.outputs() of each stream as <path>/stream<k>_<name>.npy, streams in order while the total stays within
+    DUMP_BYTES_MAX (a config-4 stream is about 1.5 MB, so every stream of a default run fits)."""
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for cs in cams:
+        arrays = cs.outputs()
+        size = sum(a.nbytes for a in arrays.values())
+        if total + size > DUMP_BYTES_MAX:
+            break
+        for name, a in arrays.items():
+            np.save(os.path.join(path, "stream%d_%s.npy" % (cs.sid, name)), a)
+        total += size
 
 
 def run_ours(args):
@@ -458,16 +505,11 @@ def run_ours(args):
         if errs:
             raise errs[0]
 
-    event_ms, fps_info = {}, {}
+    event_ms = {}
+    fps = args.frames_per_step
 
     def timed(name, steps, warmup, offset):
-        # warm-up (>= 3 frames per stream), also calibrates frames_per_step so that the timed region lasts >= ~2 s
-        t0 = time.perf_counter()
-        run_all(name, offset, offset + warmup)
-        torch.cuda.synchronize()
-        per_frame = max_over_ranks((time.perf_counter() - t0) / warmup, dev, world)
-        fps = args.frames_per_step if args.frames_per_step > 0 else int(min(500, max(1, np.ceil(args.min_seconds / (steps * per_frame)))))
-        fps_info[name] = fps
+        run_all(name, offset, offset + warmup * fps)
         for cs in cams:
             cs.reset()
         barrier()
@@ -477,7 +519,7 @@ def run_ours(args):
         e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
         e0.record()
         t0 = time.perf_counter()
-        run_all(name, offset + warmup, offset + warmup + steps * fps)
+        run_all(name, offset + warmup * fps, offset + (warmup + steps) * fps)
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
         e1.record(); e1.synchronize()
@@ -491,10 +533,12 @@ def run_ours(args):
     t_dev, launches = timed("step_device", args.steps, args.warmup, 0)
     dev_state = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in cams[0].st_dev.items()}   # per-kernel times: stream 0
     dev_stage = cams[0].stage_ms["device"].copy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(cams, args.dump_outputs)
     t_e2e, _ = timed("step_host", args.steps, args.warmup, 7)
     host_stage = cams[0].stage_ms["host"].copy()
     clocks = sampler.stop() if sampler else None
-    fps_d, fps_h = fps_info["step_device"], fps_info["step_host"]
+    fps_d = fps_h = fps
 
     # ---- per-frame latency of ONE stream alone on the GPU (what a live SLAM session sees): spin waits, the BA iteration
     #      replayed as a CUDA graph.  Reported next to the throughput figures, not part of `value`.
@@ -566,9 +610,8 @@ def run_ours(args):
             "dtype": "u8 (extract, Hamming) + f64 (pose optimiser, local BA)", "data": "synthetic (seeded numpy frames and BA graph; no datasets offline)",
             "config": {"workload": cfg["name"], "streams_per_gpu": S, "frames_per_step_per_stream": fps_d, "lm_speculation_width": spec, "lm_second_batch_width": spec2, "lm_cuda_graphs": bool(args.graphs), "ba_solver_cluster_ctas": cluster if cfg["ba"] else None, "host_wait": wait,
                        "host_cores": host_cores(),
-                       "step": "%d frame(s) on each of the %d independent camera streams of a GPU (own handles and CUDA streams, one host thread each); "
-                               "the driver's step count is kept, frames per step are calibrated in the warm-up so that the timed region lasts >= %.1f s"
-                               % (fps_d, S, args.min_seconds),
+                       "step": "%d frame(s) on each of the %d independent camera streams of a GPU (own handles and CUDA streams, one host thread each)"
+                               % (fps_d, S),
                        "l2": "frame ring of %d x %.2f MB = %.0f MB > 126 MB L2" % (ring, W * H / 1e6, ring * W * H / 1e6),
                        "value_path": "whole path, inputs resident in HBM (extract_device, brute_force_match_device, frame_index_create_device, "
                                      "local_ba_prepare_device / run / fetch_device); the projection matcher's landmark arrays and the pose "
@@ -784,8 +827,8 @@ def main():
     ap.add_argument("--config", type=int, default=4, choices=sorted(CONFIGS), help="BASELINE.json configs[n-1]; 4 = the metric's configuration")
     ap.add_argument("--ring", type=int, default=0, help="frames in the device ring (0: just above 126 MB, the L2 size)")
     ap.add_argument("--streams", type=int, default=0, help="independent camera streams per GPU (0: the config's default, 8; config 5: 1)")
-    ap.add_argument("--frames-per-step", type=int, default=0, help="frames per stream per step (0: calibrated so that the timed region lasts --min-seconds)")
-    ap.add_argument("--min-seconds", type=float, default=2.0)
+    ap.add_argument("--frames-per-step", type=int, default=8,
+                    help="frames per stream per step (default 8: the default 20 steps then time 160 frames on each stream)")
     ap.add_argument("--spec", type=int, default=0, help="local BA speculation width 1..4 (0 = default 4)")
     ap.add_argument("--spec2", type=int, default=0, help="local BA: width of a statically enqueued second trial batch (0 = none)")
     ap.add_argument("--graphs", action="store_true", help="local BA: replay the Levenberg iteration as a CUDA graph in the throughput legs too (default: only in the single-stream latency pass)")
@@ -796,7 +839,11 @@ def main():
     ap.add_argument("--no-latency", action="store_true", help="skip the single-stream latency pass")
     ap.add_argument("--cpu-budget", type=float, default=20.0)
     ap.add_argument("--ref-threads", type=int, default=0, help="CPU arm: independent streams (0 = one per usable host core, cgroup quota respected)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the value leg returned for the last frame of each camera stream as DIR/*.npy")
     args = ap.parse_args()
+    if args.frames_per_step < 1:
+        ap.error("--frames-per-step must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     out = run_reference(args) if args.impl == "reference" else run_ours(args)
     if out is not None:
